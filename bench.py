@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- STEP inference throughput (clips/s) on B200, BASELINE.json config 4.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic clips: I3D trunk -> (ROIAlign ->
 two-branch head -> tube update) x max_iter=3, B=8 clips per GPU, T=32, 224x224, 11 proposals/clip,
@@ -18,6 +18,8 @@ roofline : the dominant kernel class (conv_umma_kernel, tcgen05 implicit GEMM): 
 cpu_baseline : the oracle port (oracle/model.py, torch-CPU fp32 == the reference's arithmetic) on
         this box's host cores on a bounded sample (1 clip per timed pass).
 --impl reference : the same oracle timed as the reference arm (its own CPU implementation of the path).
+--dump-outputs DIR : after the K timed steps, the outputs of the last one as .npy files (see dump_outputs); the inputs
+        are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -116,11 +118,22 @@ def build_nets(cfg, device):
     return nets
 
 
+def workload(rank):
+    """cfg, clips [B, T_in, 3, HW, HW] (host) and proposals of the measured workload: rank r owns clips [r*B, (r+1)*B) of
+    the synthetic stream (different seed per rank)."""
+    from step_b200 import synth
+    W = WORKLOAD
+    cfg = synth.make_cfg(fp16=True, T=W["T_in"] // 4, max_iter=W["max_iter"], NUM_CHUNKS={1: 1, 2: 1, 3: 1},
+                         image_size=(W["HW"], W["HW"]))
+    clips = synth.make_clips(W["B"], W["T_in"], W["HW"], W["HW"], seed=1234 + rank)
+    return cfg, clips, synth.make_proposals(W["B"], W["N"], cfg.T, W["HW"], W["HW"])
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
     import step_b200
-    from step_b200 import _lib, engine, synth
+    from step_b200 import _lib, engine
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -132,14 +145,11 @@ def run_ours(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     W = WORKLOAD
-    cfg = synth.make_cfg(fp16=True, T=W["T_in"] // 4, max_iter=W["max_iter"], NUM_CHUNKS={1: 1, 2: 1, 3: 1},
-                         image_size=(W["HW"], W["HW"]))
+    cfg, clips_host, tubes = workload(rank)
     nets = build_nets(cfg, dev)
     B = W["B"]
-    # rank r owns clips [r*B, (r+1)*B) of the synthetic stream (different seed per rank)
-    clips_host = synth.make_clips(B, W["T_in"], W["HW"], W["HW"], seed=1234 + rank).pin_memory()
+    clips_host = clips_host.pin_memory()
     clips_dev = clips_host.to(dev)
-    tubes = synth.make_proposals(B, W["N"], cfg.T, W["HW"], W["HW"])
     cap = min(DETECT["topk"], W["N"] * cfg.num_classes)
     # what leaves the GPU per step: the kept detections of every clip {x1,y1,x2,y2,score,class,tube,0} and their count
     out_host = {"det": torch.empty((B, cap, 8), dtype=torch.float32).pin_memory(),
@@ -198,8 +208,9 @@ def run_ours(args):
         cur = torch.cuda.current_stream(dev)
         streams[i].wait_stream(cur)
         with torch.cuda.stream(streams[i]):
-            runners[i](x)
+            step.hist = runners[i](x)
             last = runners[i].detections[cfg.max_iter - 1]     # per-class NMS + top-k ran inside the captured step
+        step.det = last
         step.last_stream = streams[i]
         if n_run == 1:
             cur.wait_stream(streams[i])
@@ -257,6 +268,8 @@ def run_ours(args):
     mark("warm-up enqueued")
     ms = timed(lambda: step(clips_dev), args.steps)
     mark("device-resident region timed")
+    if args.dump_outputs and rank == 0:     # before later steps reuse the runners' static output buffers
+        dump_outputs(args.dump_outputs, step.hist, step.det, gather)
     launches = launches_per_step * args.steps
 
     # Insurance for the measured number: should the end-to-end region ever fail to drain (seen with programmatic dependent
@@ -398,6 +411,44 @@ def run_ours(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, hist, det, gather):
+    """Writes what one step hands its caller to out_dir/<name>.npy (float32), so that two builds can be compared output
+    for output on the same seeded inputs: per refinement step k the `inference` history entry (step<k>_pred_prob
+    [R, classes] -- the same scores on every frame --, step<k>_pred_loc [R, T, 4] and, in temporal-predict mode, the
+    neighbour boxes), then the kept detections det [B, cap, 8] and their counts [B]; with several GPUs also the
+    detections gathered from every rank [ranks, B, cap * 8 + 1].  Detection rows at or past a clip's count are written
+    as zeros: the step does not write them, they hold whatever an earlier step left in the buffer."""
+    import numpy as np
+
+    def blank_unwritten(d, count):   # d [clips, cap, 8], count [clips]
+        d[np.arange(d.shape[1])[None, :] >= count[:, None]] = 0.0
+    out = {}
+    for k, h in enumerate(hist):
+        out["step%d_pred_prob" % k] = h["pred_prob"][:, 0]
+        for name in ("pred_loc", "pred_first_loc", "pred_last_loc"):
+            if h[name] is not None:
+                out["step%d_%s" % (k, name)] = h[name]
+    out["det"], out["count"] = det["det"], det["count"]
+    if gather is not None:
+        out["gathered"] = gather
+    arrays = {k: v.detach().float().cpu().numpy().copy() for k, v in out.items()}
+    blank_unwritten(arrays["det"], arrays["count"])
+    if gather is not None:
+        g = arrays["gathered"]
+        d = g[..., :-1].reshape(-1, arrays["det"].shape[1], 8)
+        blank_unwritten(d, g[..., -1].reshape(-1))
+        g[..., :-1] = d.reshape(g.shape[:-1] + (-1,))
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def timed_local(torch, fn, steps):
@@ -567,16 +618,15 @@ def run_reference(args):
     import torch
     cores = host_threads()        # times a warm-up pass per candidate thread count and keeps the faster
     torch.set_num_threads(cores)
-    steps = min(args.steps, 5)
-    t = sum(oracle_pass(1) for _ in range(steps))
-    v = round(steps / t, 4)
+    t = sum(oracle_pass(1) for _ in range(args.steps))
+    v = round(args.steps / t, 4)
     print(json.dumps({
         "impl": "reference", "metric": "clips/sec (T=32,224x224) STEP max_iter=3", "value": v, "unit": "clips/s",
-        "n_gpus": args.gpus, "steps": steps, "warmup": min(args.warmup, 1), "ms_per_step": round(t / steps * 1e3, 2),
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": min(args.warmup, 1), "ms_per_step": round(t / args.steps * 1e3, 2),
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": "C4 shape, bounded sample: 1 clip per step (T=32, 224x224, 11 proposals, max_iter=3)"},
         "cpu_baseline": {"value": v, "unit": "clips/s", "cores": cores, "kind": "port",
-                         "sample": "1 clip per step, %d steps" % steps},
+                         "sample": "1 clip per step, %d steps" % args.steps},
         "e2e": {"value": v, "unit": "clips/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
 
@@ -584,14 +634,23 @@ def run_reference(args):
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=250, help="timed steps (default: ~1 s of device time)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 250 for ours, ~1 s of device time; 5 for reference, one clip per step)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--skip-cpu", action="store_true", help="omit the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying the CUDA graph")
     ap.add_argument("--inflight", type=int, default=3, help="independent batches kept in flight on separate streams")
     ap.add_argument("--verbose", action="store_true", help="phase markers on stderr (to locate a stall)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32; rank 0)")
     a = ap.parse_args()
+    if a.steps is None:
+        a.steps = 250 if a.impl == "ours" else 5
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         run_reference(a)

@@ -11,8 +11,7 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu under gpurun)")
-    config.addinivalue_line("markers", "refonly: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "gpu: needs a real B200 (select with -m gpu)")
 
 
 @pytest.fixture(scope="session")

@@ -2,6 +2,7 @@
 never imports the oracle; no compute calls are made here (no GPU in this tier)."""
 import os
 import re
+import shutil
 import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -27,7 +28,10 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_library_is_sm100a_native():
-    out = subprocess.run(["cuobjdump", "-lelf", os.path.join(ROOT, "step_b200", "libstep_b200.so")],
+    from step_b200 import build
+    # the toolkit that built the library, also when its bin/ is not on PATH
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(build.NVCC), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", os.path.join(ROOT, "step_b200", "libstep_b200.so")],
                          capture_output=True, text=True).stdout
     assert "sm_100a" in out
 

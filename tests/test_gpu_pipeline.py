@@ -446,14 +446,41 @@ def test_bench_with_three_batches_in_flight_completes():
     """bench.py's measured configuration (CUDA graphs, three batches in flight on separate streams) runs to completion and
     prints its JSON line.  A kernel that only works when it has the GPU to itself shows up here as a timeout: an
     experimental variant of the fused bottleneck exit passed every single-stream test and stalled exactly this run
-    (tools/experiments/README.md)."""
+    (tools/experiments/README.md).  What --dump-outputs writes equals one eager step on the same seeded inputs."""
     import json
     import os
     import subprocess
     import sys
+    import tempfile
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "40", "--warmup", "3", "--skip-cpu"],
-                       capture_output=True, text=True, timeout=240, cwd=root)
-    assert r.returncode == 0, r.stderr[-2000:]
-    j = json.loads(r.stdout.strip().splitlines()[-1])
-    assert j["config"]["batches_in_flight"] == 3 and j["value"] > 0 and j["gpu_launches"] > 0
+    with tempfile.TemporaryDirectory() as td:
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "40", "--warmup", "3", "--skip-cpu",
+                            "--dump-outputs", td], capture_output=True, text=True, timeout=240, cwd=root)
+        assert r.returncode == 0, r.stderr[-2000:]
+        j = json.loads(r.stdout.strip().splitlines()[-1])
+        assert j["config"]["batches_in_flight"] == 3 and j["value"] > 0 and j["gpu_launches"] > 0
+        # the last timed step's outputs: 8 clips x 11 proposals, 60 classes, 3 refinement steps, the kept detections
+        det, count = np.load(os.path.join(td, "det.npy")), np.load(os.path.join(td, "count.npy"))
+        prob = np.load(os.path.join(td, "step2_pred_prob.npy"))
+        assert det.dtype == count.dtype == prob.dtype == np.float32
+        assert prob.shape == (88, 60) and np.isfinite(prob).all() and det.shape[0] == count.shape[0] == 8
+        assert count.sum() > 0 and (count <= det.shape[1]).all()
+        # ... and they are what one eager step of the same workload computes, bit for bit
+        import importlib.util
+        import step_b200
+        spec = importlib.util.spec_from_file_location("bench", os.path.join(root, "bench.py"))
+        bench = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(bench)
+        cfg, clips, tubes = bench.workload(0)
+        W = bench.WORKLOAD
+        runner = step_b200.StepRunner(cfg, bench.build_nets(cfg, torch.device("cuda", 0)), W["B"], W["T_in"], W["HW"], W["HW"],
+                                      tubes, use_graph=False, detect=bench.DETECT)
+        with torch.no_grad():
+            hist = runner(clips.cuda())
+        torch.cuda.synchronize()
+        eager = os.path.join(td, "eager")
+        bench.dump_outputs(eager, hist, runner.detections[cfg.max_iter - 1], None)
+        names = sorted(n for n in os.listdir(td) if n.endswith(".npy"))
+        assert names == sorted(os.listdir(eager)) and "step2_pred_loc.npy" in names
+        for n in names:
+            assert np.array_equal(np.load(os.path.join(td, n)), np.load(os.path.join(eager, n))), n

@@ -74,22 +74,38 @@ def test_oracle_same_pad_table():
     assert E.same_pad(7, 2) == (2, 3) and E.same_pad(1, 1) == (0, 0)
 
 
-@pytest.mark.refonly
-def test_compat_patch_substitutes_the_names_the_reference_drivers_import():
-    """Build container only (needs /root/reference): after compat.patch(<reference root>) the reference's own import
-    lines (test.py:19-25) resolve to step_b200, and its utils.utils.inference IS ours -- without editing a reference file."""
-    import os
+# The part of the reference tree its drivers' import lines (test.py:19-25) reach: a `models` package, `utils/utils.py`
+# (the progressive `inference`, which imports its helpers from `utils/tube_utils.py`) and `utils/tube_utils.py`.  The
+# stand-in below has that layout; importing its `models` package or calling any of its functions fails.
+STAND_IN_REFERENCE = {
+    "models/__init__.py": "raise ImportError('the stand-in reference models package was imported')\n",
+    "utils/__init__.py": "",
+    "utils/tube_utils.py": "".join("def %s(*args, **kwargs):\n    raise AssertionError('stand-in')\n\n\n" % n for n in (
+        "compute_box_iou", "compute_tube_iou", "decode_coef", "extrapolate_tubes", "flatten_tubes", "valid_tubes")),
+    # the helpers the reference's utils/utils.py takes from utils.tube_utils at import time (utils.py:13)
+    "utils/utils.py": ("from utils.tube_utils import (compute_tube_iou, decode_coef, extrapolate_tubes, flatten_tubes,\n"
+                       "                              valid_tubes)\n"
+                       "\n\ndef inference(args, conv_feat, context_feat, nets, exec_iter, tubes):\n"
+                       "    raise AssertionError('the stand-in reference inference ran')\n"),
+}
+
+
+def test_compat_patch_substitutes_the_names_the_reference_drivers_import(tmp_path):
+    """After compat.patch(<reference root>) the reference's own import lines (test.py:19-25) resolve to step_b200, and
+    its utils.utils.inference IS ours -- without editing a reference file.  Runs on a stand-in tree with the reference's
+    module layout, so that a `models` package in the tree must lose to ours."""
     import sys
-    if not os.path.isdir("/root/reference/models"):
-        pytest.skip("reference tree not present")
     import step_b200
     import step_b200.compat as compat
+    for rel, text in STAND_IN_REFERENCE.items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(text)
     saved = dict(sys.modules)
     saved_path = list(sys.path)
     try:
         for k in [k for k in sys.modules if k == "models" or k.startswith("models.") or k.startswith("external") or k == "utils" or k.startswith("utils.")]:
             del sys.modules[k]
-        compat.patch("/root/reference")
+        compat.patch(str(tmp_path))
         ns = {}
         exec("from models import BaseNet, ROINet, TwoBranchNet, ContextNet\n"
              "from external.maskrcnn_benchmark.roi_layers import nms\n"
@@ -98,6 +114,7 @@ def test_compat_patch_substitutes_the_names_the_reference_drivers_import():
         assert ns["BaseNet"] is step_b200.BaseNet and ns["TwoBranchNet"] is step_b200.TwoBranchNet
         assert ns["nms"] is step_b200.roi_layers.nms and ns["inference"] is step_b200.inference
         assert ns["valid_tubes"].__module__ == "utils.tube_utils"                    # host helpers stay the reference's own
+        assert sys.modules["utils.tube_utils"].__file__.startswith(str(tmp_path))
         cfg = __import__("step_b200.synth", fromlist=["x"]).make_cfg()
         net = ns["TwoBranchNet"](cfg)
         net.load_state_dict(__import__("step_b200.synth", fromlist=["x"]).head_state_dict(100, cfg), strict=True)
