@@ -18,6 +18,7 @@
  *   conv / pool / linear / head_*   the torch.nn calls of models/i3dpt.py:43-163,
  *                  models/networks.py:69-83, models/two_branch.py:60-111,132-138,223-274,337
  *   clip_*         the permute + (apex) cast at models/networks.py:77
+ *   frames_*       data/augmentations.py:68-169,601-615; data/ava.py:330-338
  *
  * Tensor conventions: activations are channels-last -- [N, T, H, W, C] ("NDHWC") with an explicit
  * channel stride `ld` (elements) so a kernel can read or write a channel slice of a wider buffer
@@ -144,6 +145,22 @@ int step_clip_to_ndhwc(const float* clip, int N, int T, int Cc, int H, int W, vo
  * out [N,T/2,H/2,W/2,ld] f16 with channel = ((rt*2+rh)*2+rw)*Cc + c. T,H,W must be even. */
 int step_clip_to_s2d_f16(const float* clip, int N, int T, int Cc, int H, int W, void* out, int ld,
                          step_stream_t stream);
+/* Test-time input transform from decoded frames (BaseTransform, augmentations.py:601-615, then the BGR -> RGB swap and
+ * permute of ava.py:330-338): ConvertFromInts(scale) -> cv2.resize INTER_LINEAR on fp32 to (W, H) -> (v - mean) / std, in
+ * the reference's fp32 order.  frames [N,T,Hmax,Wmax,3] uint8 BGR as cv2.imread returns them; clip n fills the top-left
+ * H0 x W0 of each of its frame slots (row pitch Wmax*3 bytes), with sizes [N,2] = (H0, W0) a DEVICE int32 table, so one
+ * captured graph serves any mix of source sizes up to (Hmax, Wmax).  The caller validates the table (1 <= H0 <= Hmax,
+ * 1 <= W0 <= Wmax); the kernels clamp to the slot.  mean_* / std_* are in BGR order, as BaseTransform takes them;
+ * scale is 0 ([0,255]), 1 ([0,1]) or 2 ([-1,1]).
+ * step_frames_to_clip_f32: out [N,T,3,H,W] fp32 RGB, the clip BaseNet.forward receives.
+ * step_frames_to_s2d_f16: out [N,T/2,H/2,W/2,32] f16 (32-byte aligned), bit-identical to step_clip_to_s2d_f16(ld = 32)
+ * applied to the clip form.  T, H, W must be even. */
+int step_frames_to_clip_f32(const uint8_t* frames, const int32_t* sizes, int N, int T, int Hmax, int Wmax, int H, int W,
+                            int scale, float mean_b, float mean_g, float mean_r, float std_b, float std_g, float std_r,
+                            float* out, step_stream_t stream);
+int step_frames_to_s2d_f16(const uint8_t* frames, const int32_t* sizes, int N, int T, int Hmax, int Wmax, int H, int W,
+                           int scale, float mean_b, float mean_g, float mean_r, float std_b, float std_g, float std_r,
+                           void* out, step_stream_t stream);
 /* channels-last [M, C] (stride ld) <-> planar [N, C, S] fp32, M = N*S (boundary conversions). */
 int step_nhwc_to_nchw_f32(const void* in, int dtype, int N, int S, int C, int ld, float* out,
                           step_stream_t stream);

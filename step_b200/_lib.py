@@ -57,6 +57,8 @@ def _declare(lib):
         "step_tube_update_f32": ([P, P, P, P, P, I, I, I, I, I, Fl, Fl, P, P, P, P, S], c_int),
         "step_clip_to_ndhwc": ([P, I, I, I, I, I, P, I, I, S], c_int),
         "step_clip_to_s2d_f16": ([P, I, I, I, I, I, P, I, S], c_int),
+        "step_frames_to_clip_f32": ([P, P, I, I, I, I, I, I, I, Fl, Fl, Fl, Fl, Fl, Fl, P, S], c_int),
+        "step_frames_to_s2d_f16": ([P, P, I, I, I, I, I, I, I, Fl, Fl, Fl, Fl, Fl, Fl, P, S], c_int),
         "step_nhwc_to_nchw_f32": ([P, I, I, I, I, I, P, S], c_int),
         "step_nchw_to_nhwc": ([P, I, I, I, P, I, I, S], c_int),
         "step_conv3d_fwd": ([ctypes.POINTER(ConvParams), S], c_int),

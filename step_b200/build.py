@@ -13,11 +13,11 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libstep_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-SOURCES = ["api.cu", "nms.cu", "roi.cu", "tubes.cu", "pool_layout.cu", "conv_simt.cu", "conv_umma.cu", "conv_halo.cu", "bottleneck_exit.cu", "train.cu"]
+SOURCES = ["api.cu", "nms.cu", "roi.cu", "tubes.cu", "pool_layout.cu", "conv_simt.cu", "conv_umma.cu", "conv_halo.cu", "bottleneck_exit.cu", "train.cu", "frames.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC", "--use_fast_math=false" if False else "-Xptxas", "-v"]
-# nms/roi/tubes rely on explicitly rounded intrinsics; -fmad=false additionally forbids contraction
-NO_FMAD = {"nms.cu", "roi.cu", "tubes.cu", "train.cu"}
+# nms/roi/tubes/frames rely on explicitly rounded intrinsics; -fmad=false additionally forbids contraction
+NO_FMAD = {"nms.cu", "roi.cu", "tubes.cu", "train.cu", "frames.cu"}
 
 
 def _deps(src):

@@ -136,14 +136,23 @@ class BaseNet(nn.Module):
             # stride-2 stem as a stride-1 4x4x4 filter over the space-to-depth clip (engine.pack_stem_s2d)
             s2d = Act.empty(N, T // 2, H // 2, W // 2, 32, L.F16, x.device)
             L.check(L.lib().step_clip_to_s2d_f16(L.ptr(src), N, T, C, H, W, L.ptr(s2d.buf), 32, L.stream()))
-            a = m[0].forward_s2d(s2d)
-        else:
-            if code == L.F16:
-                raise RuntimeError("BaseNet(fp16): T, H, W must be even and C == 3")
-            cp = (C + 3) // 4 * 4
-            a = Act.empty(N, T, H, W, cp, code, x.device)
-            L.check(L.lib().step_clip_to_ndhwc(L.ptr(src), N, T, C, H, W, L.ptr(a.buf), code, cp, L.stream()))
-            a = m[0](a)
+            return self.forward_s2d(s2d)
+        if code == L.F16:
+            raise RuntimeError("BaseNet(fp16): T, H, W must be even and C == 3")
+        cp = (C + 3) // 4 * 4
+        a = Act.empty(N, T, H, W, cp, code, x.device)
+        L.check(L.lib().step_clip_to_ndhwc(L.ptr(src), N, T, C, H, W, L.ptr(a.buf), code, cp, L.stream()))
+        return self._after_stem(m[0](a))
+
+    def forward_s2d(self, s2d):
+        """fp16 trunk from the stem's space-to-depth input, an Act [N, T/2, H/2, W/2, 32] (step_clip_to_s2d_f16's layout,
+        or step_frames_to_s2d_f16 straight from decoded frames)."""
+        if not self.fp16:
+            raise RuntimeError("BaseNet.forward_s2d: the space-to-depth stem is the fp16 path")
+        return self._after_stem(self.base_model[0].forward_s2d(s2d))
+
+    def _after_stem(self, a):
+        m = self.base_model
         for i in range(1, len(m)):
             a = m[i](a)
         return a
